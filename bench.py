@@ -12,6 +12,7 @@ step     : zero grad -> ONE fused pair kernel (gather + distance + loss + gradie
            push the new rows to every rank) -- NCCL reduce-scatter / all-gather only if CUDA IPC is unavailable.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--pairs-log2 24] [--nodes 2000000]
+                  [--dump-outputs DIR]
 
 `value`  : whole-job pairs/s with the pair batches resident in HBM (CUDA events, max over ranks).
 `e2e`    : same metric through the public API from PINNED HOST buffers.  Sampled path: the step's input is its 1024
@@ -34,6 +35,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -47,6 +49,7 @@ METRIC = 'spd4_pair_dist_grad_evals_per_sec'
 UNIT = 'pairs/s'
 BYTES_PER_PAIR = 4 * 16 * 4 + 4 + 8  # SURVEY 8(d): 2 endpoint reads + 2 gradient accumulations + target + 2 indices
 N_SOURCES = 1024
+DUMP_ROWS = 1 << 18  # --dump-outputs: 16 MB of the 128 MB point table
 
 
 def parse():
@@ -92,7 +95,16 @@ def parse():
     ap.add_argument('--workload', default='5', help="'5' (default, the bench line) or one of 1, 2a, 2b, 3a, 3b, 4 (or a "
                     "comma list / 'all'): epoch time of that BASELINE config -- on the GPU through TrainingEngine, or "
                     "with --impl reference on the host CPU")
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last device-resident timed step returned as '
+                    'DIR/<name>.npy: loss.npy (float64, the step loss) and points.npy (float32, the updated SPD 4x4 '
+                    f'points of a fixed, seeded sample of min(N, {DUMP_ROWS}) rows in ascending row order), so that '
+                    'two builds run with the same arguments can be compared output for output.  The inputs are the '
+                    'same on every run; the gradient is summed with atomics, so two runs agree to summation order, '
+                    'not bit for bit')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -463,9 +475,9 @@ def gpu_config_epoch(tag, epochs, dev, with_cpu=True):
             opt = RiemannianSGD(emb.xs, lr=0.01, max_grad_norm=20, exact=True)   # run_grid.py:30-33
         else:
             opt = RiemannianAdam(emb.xs, lr=0.01, max_grad_norm=100, exact=True)  # run_grid.py:25-28
-        os.makedirs('/tmp/bench_configs', exist_ok=True)
+        save_dir = tempfile.TemporaryDirectory(prefix='bench_configs_')
         eng = TrainingEngine(embedding=emb, optimizer=opt, objective_fn=QuotientLoss(), n_epochs=epochs, alpha=1.0,
-                             batch_size=batch_nodes, tensorboard=False, save_dir='/tmp/bench_configs')
+                             batch_size=batch_nodes, tensorboard=False, save_dir=save_dir.name)
         kernel_events, epoch_ms = [], []
 
         def timed(fn):
@@ -498,6 +510,7 @@ def gpu_config_epoch(tag, epochs, dev, with_cpu=True):
             _ops.pairs_loss_fused, _ops.pairs_dist2, _ops.pairs_grad = saved
         launches = L.launch_count() - launches0
         final_loss = float(eng.writer.history['quotient_loss'][-1][1])
+        save_dir.cleanup()
     finally:
         torch.set_default_device(prev_dev)
     bs = n if batch_nodes is None else min(n, batch_nodes)
@@ -577,6 +590,15 @@ def bfs_secondary(graph, n_nodes, dev, reps=5):
                          'frac': alg / (ms * 1e-3) / 1e9 / peak, 'algorithmic_bytes_per_call': alg,
                          'basis': 'level matrix written once + per level: CSR read, frontier words read, visited and '
                                   'next words updated'}}
+
+
+def output_snapshot(trainer, loss, n_points, sharded):
+    """--dump-outputs: host copies of what the step handed back -- its loss and the updated point table, of which a
+    fixed sample of rows (the same rows on every run) keeps the dump small.  Row-sharded: every rank must call it."""
+    x = trainer.gather() if sharded else trainer.emb.xs[0].detach()
+    rows = torch.randperm(n_points, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    return {'loss': loss.detach().double().reshape(1).cpu().numpy(),
+            'points': x.index_select(0, rows.to(x.device)).float().cpu().numpy()}
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -692,6 +714,8 @@ def main():
         loss = trainer.step(*dev_batches[k % len(dev_batches)], epoch=1, segments=seg)
     t1.record()
     barrier()
+    # taken before the steps below move the points on
+    outputs = output_snapshot(trainer, loss, N, sharded) if args.dump_outputs and (rank == 0 or sharded) else None
     nvlink = None
     if nvl:  # NVLink payload bytes per step, from the driver's counters, over a few extra (untimed) steps
         nvl.start()
@@ -770,6 +794,10 @@ def main():
         if pg is not None:
             torch.distributed.destroy_process_group()
         return
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, f'{name}.npy'), a)
 
     peak, peak_src = hbm_peak()
     achieved = P * BYTES_PER_PAIR / (pair_ms * 1e-3) / 1e9

@@ -84,23 +84,6 @@ def test_optimizer_trajectories(name, oname, tag):
             assert rel_err(state[key], g[f'{oname}_{key}']) < TOL[tag] * 50
 
 
-def test_live_reference_if_present():
-    """In the build container also compare against the imported reference on fresh random inputs."""
-    import ref_import
-    if not ref_import.available():
-        pytest.skip('reference tree not present (GPU box)')
-    ref_import.load()
-    from graphembed.manifolds import SymmetricPositiveDefinite, Lorentz
-    torch.manual_seed(123)
-    for n in (2, 3, 5):
-        ref = SymmetricPositiveDefinite(n)
-        x = ref.rand(9, ir=0.5).double()
-        assert rel_err(O.SpdOracle(n).pdist2(x), ref.pdist(x, squared=True)) < 1e-12
-    ref = Lorentz(6)
-    x = ref.rand(9, ir=0.5).double()
-    assert rel_err(O.LorentzOracle(6).pdist2(x), ref.pdist(x, squared=True)) < 1e-12
-
-
 # ---- objectives / metrics / epoch loop added with the TrainingEngine row (SURVEY 8f-1, 8f-2) ------------------------
 @pytest.mark.parametrize('tag', ['f64', 'f32'])
 def test_kl_sne_and_metrics_vs_reference(tag):
