@@ -371,8 +371,19 @@ GM_HD bool jacobi_eigh(T (&a)[N * N], T (&v)[N * N], T (&w)[N], int max_sweeps =
     T apq = a[p * N + q];
     T t, c, s;
     Num<T>::rotation(a[q * N + q] - a[p * N + p], apq, t, c, s);
-    a[p * N + p] = Num<T>::fma(-t, apq, a[p * N + p]);
-    a[q * N + q] = Num<T>::fma(t, apq, a[q * N + q]);
+    if constexpr (N >= 5) {
+      // The diagonal from the same rounded (c, s) that rotates the off-diagonal rows below.  The cheaper
+      // a_pp - t a_pq assumes the exact rotation; with the rounded one it is not a congruence, and on spectra over
+      // 4 decades (6x6 fp32, condition up to 1e8) that mismatch biases every eigenvalue sum inward: d2 -1.1e-5 on
+      // average, the loss summed over such pairs 1.4e-5 low (tests/test_gpu_spd_hotpath.py, class C), against
+      // 3e-8 with this form.  n <= 4 keep a_pp - t a_pq: there the same bars hold and it is the bench.py path.
+      const T app = a[p * N + p], aqq = a[q * N + q], cs2 = (T)2 * c * s * apq;
+      a[p * N + p] = c * c * app - cs2 + s * s * aqq;
+      a[q * N + q] = s * s * app + cs2 + c * c * aqq;
+    } else {
+      a[p * N + p] = Num<T>::fma(-t, apq, a[p * N + p]);
+      a[q * N + q] = Num<T>::fma(t, apq, a[q * N + q]);
+    }
     a[p * N + q] = (T)0;
     a[q * N + p] = (T)0;
     GM_UNROLL for (int r = 0; r < N; ++r) {
