@@ -197,8 +197,7 @@ int gm_product_loss(int32_t dtype, int32_t F, const void* const* d2_ptrs_host, c
  * Host arrays of length F: mans, x, grad, sp.  Pairs / targets as gm_pairs_loss_fused (LIST / TRIU / SAMPLED; every
  * target mode).  Supported products: at most one SPD factor (either divergence) and up to three of Lorentz / Sphere /
  * Euclidean, 2 <= F <= 4, one dtype; anything else returns GM_EUNSUPPORTED and the caller keeps the unfused sequence
- * gm_pairs_dist2 x F -> gm_product_loss -> gm_pairs_grad x F.  gm_train_epoch_product uses it when it can
- * (GM_PRODUCT_FUSED=0 in the environment forces the unfused sequence). */
+ * gm_pairs_dist2 x F -> gm_product_loss -> gm_pairs_grad x F.  gm_train_epoch_product uses it when it can. */
 int gm_pairs_product_fused(int32_t F, const gm_manifold_t* mans, void* const* x, const gm_pairs_t* pairs,
                            const gm_targets_t* targets, const gm_loss_t* loss, const double* sp, double* acc,
                            void* const* grad, gm_stream_t stream);

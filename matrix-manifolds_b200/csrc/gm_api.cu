@@ -174,38 +174,109 @@ static int pair_dispatch(const PairArgs& a) {
   return vec_launch(a);
 }
 
-// ---------------------------------------------------------------------------
-// product-manifold loss over F distance vectors
-// ---------------------------------------------------------------------------
-template <typename T>
-__global__ void __launch_bounds__(256)
-product_loss_kernel(int F, FactorPtrs fp, TargetSpec tg, PairSpec ps, LossCfg lc, long long P,
-                    double* __restrict__ acc, T* __restrict__ out_g) {
-  __shared__ double red[8];
-  long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  bool active = k < P;
-  double lv = 0.0;
-  double gd[8];
-  for (int f = 0; f < 8; ++f) gd[f] = 0.0;
-  if (active) {
-    // sum() of a Python list starts from int 0 and adds left to right (modules.py:84-88)
-    T m = (T)0;
-    T d2[8];
-    for (int f = 0; f < F; ++f) {
-      d2[f] = ((const T*)fp.d2[f])[k];
-      T term = (T)fp.sp[f] * d2[f];
-      m = (f == 0) ? term : m + term;
-    }
-    long long ra = 0, rb = 0;
-    if (tg.mode == GM_TGT_DENSE) decode_pair(ps, k, ra, rb);  // node ids index the dense target matrix
-    T g = fetch_target<T>(tg, k, ra, rb);
-    T dm;
-    lv = (double)loss_term<T>(lc, g, m, dm);
-    if (out_g) out_g[k] = dm;
-    for (int f = 0; f < F; ++f) gd[f] = (double)dm * (double)d2[f];
+// the loss request: QuotientLoss needs at least one of its two terms
+int check_loss(const gm_loss_t* loss) {
+  if (loss->kind != GM_LOSS_QUOTIENT && loss->kind != GM_LOSS_STRESS) return GM_EINVAL;
+  if (loss->kind == GM_LOSS_QUOTIENT && !loss->inc_l1 && !loss->inc_l2) return GM_EINVAL;
+  return GM_OK;
+}
+
+// targets of a K_FUSED request: hop counts packed into the top byte of idx_j need int32 LIST or SAMPLED pairs, drawn
+// pairs bring their hop count with them, and every other target mode reads targets->data
+static int check_fused_targets(const gm_pairs_t* pairs, const gm_targets_t* targets) {
+  if (pairs->mode == GM_PAIRS_ELEMENTWISE) return GM_EINVAL;
+  if (targets->mode < GM_TGT_VECTOR || targets->mode > GM_TGT_HOPS_PACKED) return GM_EINVAL;
+  const bool packed = targets->mode == GM_TGT_HOPS_PACKED;
+  if (packed && ((pairs->mode != GM_PAIRS_LIST && pairs->mode != GM_PAIRS_SAMPLED) || pairs->idx64)) return GM_EINVAL;
+  if (pairs->mode == GM_PAIRS_SAMPLED && !packed) return GM_EINVAL;
+  if (pairs->P > 0 && !packed && !targets->data) return GM_ENULL;
+  return GM_OK;
+}
+
+static bool optim_kind_ok(const gm_optim_t* opt) { return opt->kind == GM_OPT_RSGD || opt->kind == GM_OPT_RADAM; }
+
+// the optimizer request: RAdam needs both moment buffers and step >= 1, RSGD with momentum its momentum buffer
+static int check_optim(const gm_optim_t* opt, const void* buf1, const void* buf2) {
+  if (!optim_kind_ok(opt)) return GM_EINVAL;
+  if (opt->kind == GM_OPT_RADAM && (!buf1 || !buf2 || opt->step < 1)) return GM_EINVAL;
+  if (opt->kind == GM_OPT_RSGD && opt->has_momentum && !buf1) return GM_ENULL;
+  return GM_OK;
+}
+
+// PointArgs of `man`; with an optimizer, its step (op -1) and the state buffers that step uses
+static PointArgs point_args(const gm_manifold_t* man, const gm_optim_t* opt, void* buf1, void* buf2) {
+  PointArgs a{};
+  a.kind = man->kind; a.dtype = man->dtype; a.n = man->n; a.p = man->p; a.flags = man->flags;
+  a.wmin = man->wmin; a.wmax = man->wmax; a.c_dev = man->c_dev;
+  a.op = -1;
+  if (opt) {
+    a.oc = make_optim_cfg(opt);
+    a.grassmann_retr_qr = opt->grassmann_retr_qr;
+    a.buf1 = (opt->kind == GM_OPT_RSGD && !opt->has_momentum) ? nullptr : buf1;
+    a.buf2 = (opt->kind == GM_OPT_RADAM) ? buf2 : nullptr;
   }
-  block_accumulate(lv, acc, red);
-  for (int f = 0; f < F; ++f) block_accumulate(gd[f], acc + 1 + f, red);
+  return a;
+}
+
+// One rank's PeerTable.  phase < 0: the owner update of gm_optim_step_peer, which also reads every rank's point and
+// gradient shard; phase 0 / 1: gm_peer_barrier (phase 1 sums no per-step scalars).
+static int peer_table(const gm_peers_t* peers, int phase, PeerTable& pt) {
+  static const long long timeout_s = [] { const char* e = getenv("GM_PEER_TIMEOUT_S"); return e ? atoll(e) : 300LL; }();
+  static const int chunks = [] { const char* e = getenv("GM_PEER_CHUNKS"); return e ? atoi(e) : 4; }();
+  pt = PeerTable{};
+  pt.world = peers->world; pt.rank = peers->rank; pt.row_lo = peers->row_lo; pt.epoch = peers->epoch;
+  pt.n_acc = phase == 1 ? 0 : peers->n_acc;
+  for (int r = 0; r < peers->world; ++r) {
+    if (!peers->flags[r] || (phase < 0 && (!peers->x[r] || !peers->grad[r]))) return GM_ENULL;
+    if (pt.n_acc > 0 && !peers->acc[r]) return GM_ENULL;
+    pt.x[r] = peers->x[r]; pt.g[r] = peers->grad[r];
+    pt.flags[r] = (unsigned long long*)peers->flags[r];
+    pt.acc[r] = (const double*)peers->acc[r];
+  }
+  if (pt.n_acc > 0 && !peers->acc_out) return GM_ENULL;
+  pt.acc_out = (double*)peers->acc_out;
+  pt.gsum = peers->gsum;
+  pt.timeout_ns = timeout_s > 0 ? (unsigned long long)timeout_s * 1000000000ull : 0ull;
+  pt.chunks = chunks;
+  return GM_OK;
+}
+
+// The K_FUSED launch request shared by the fused entry points; the caller adds the point / gradient tables.
+static PairArgs fused_args(const gm_manifold_t* man, const gm_pairs_t* pairs, const gm_targets_t* targets,
+                           const gm_loss_t* loss, double scale_sp, double* acc, gm_stream_t stream) {
+  PairArgs a{};
+  fill_manifold(a, man);
+  a.kmode = K_FUSED;
+  a.ps = make_pairs(pairs);
+  a.tg = make_targets(targets);
+  if (targets->mode == GM_TGT_HOPS_PACKED) { a.tg.data = pairs->idx_j; a.ps.jmask = 0x00ffffffu; }
+  a.lc = make_loss(loss);
+  a.scale_sp = scale_sp;
+  a.acc = acc;
+  a.stream = (cudaStream_t)stream;
+  return a;
+}
+
+// The TRIU node batches of one epoch: batch k is the upper triangle of perm[i, i + b), b = batch_nodes except for the
+// last.  The walk stops at the first batch shorter than drop_last_n (or than 2 nodes); a walk longer than max_steps is
+// an error.  body(k, pairs) returns a code; *n_steps is the number of batches walked.
+template <class Body>
+static int for_each_node_batch(const void* perm, int32_t perm_is_int64, int64_t n_perm, int64_t batch_nodes,
+                               int64_t drop_last_n, int64_t max_steps, int64_t* n_steps, Body&& body) {
+  const size_t idx_bytes = perm_is_int64 ? 8 : 4;
+  int64_t k = 0;
+  for (int64_t i = 0; i < n_perm; i += batch_nodes, ++k) {
+    const int64_t b = (n_perm - i < batch_nodes) ? (n_perm - i) : batch_nodes;
+    if (b < drop_last_n || b < 2) break;
+    if (k >= max_steps) return GM_EINVAL;
+    gm_pairs_t pr{};
+    pr.mode = GM_PAIRS_TRIU; pr.idx64 = perm_is_int64; pr.P = b * (b - 1) / 2; pr.B = b;
+    pr.nodes = (const char*)perm + (size_t)i * idx_bytes; pr.k0 = 0;
+    int rc = body(k, pr);
+    if (rc) return rc;
+  }
+  *n_steps = k;
+  return GM_OK;
 }
 
 }  // namespace gm
@@ -270,26 +341,11 @@ int gm_pairs_loss_fused(const gm_manifold_t* man, const void* x, const gm_pairs_
   rc = validate_pairs(pairs);
   if (rc) return rc;
   if (!targets || !loss) return GM_ENULL;
-  if (pairs->mode == GM_PAIRS_ELEMENTWISE) return GM_EINVAL;
-  if (targets->mode < GM_TGT_VECTOR || targets->mode > GM_TGT_HOPS_PACKED) return GM_EINVAL;
-  const bool packed = targets->mode == GM_TGT_HOPS_PACKED;
-  if (packed && ((pairs->mode != GM_PAIRS_LIST && pairs->mode != GM_PAIRS_SAMPLED) || pairs->idx64)) return GM_EINVAL;
-  if (pairs->mode == GM_PAIRS_SAMPLED && !packed) return GM_EINVAL;  // drawn pairs bring their hop count with them
-  if (loss->kind != GM_LOSS_QUOTIENT && loss->kind != GM_LOSS_STRESS) return GM_EINVAL;
-  if (loss->kind == GM_LOSS_QUOTIENT && !loss->inc_l1 && !loss->inc_l2) return GM_EINVAL;
+  if ((rc = check_loss(loss)) || (rc = check_fused_targets(pairs, targets))) return rc;
   if (pairs->P == 0) return GM_OK;
-  if (!x || !acc || !grad || (!packed && !targets->data)) return GM_ENULL;
-  PairArgs a{};
-  fill_manifold(a, man);
-  a.kmode = K_FUSED;
-  a.ps = make_pairs(pairs);
+  if (!x || !acc || !grad) return GM_ENULL;
+  PairArgs a = fused_args(man, pairs, targets, loss, scale_sp, acc, stream);
   a.xa = x; a.xb = x; a.ga = grad; a.gb = grad; a.out_d2 = out_d2;
-  a.tg = make_targets(targets);
-  if (packed) { a.tg.data = pairs->idx_j; a.ps.jmask = 0x00ffffffu; }
-  a.lc = make_loss(loss);
-  a.scale_sp = scale_sp;
-  a.acc = acc;
-  a.stream = (cudaStream_t)stream;
   return pair_dispatch(a);
 }
 
@@ -306,18 +362,10 @@ int gm_pairs_loss_fused_sharded(const gm_manifold_t* man, const gm_row_shards_t*
   if (rc) return rc;
   if (!targets || !loss) return GM_ENULL;
   if (pairs->mode != GM_PAIRS_LIST && pairs->mode != GM_PAIRS_SAMPLED) return GM_EINVAL;
-  if (targets->mode < GM_TGT_VECTOR || targets->mode > GM_TGT_HOPS_PACKED) return GM_EINVAL;
-  const bool packed = targets->mode == GM_TGT_HOPS_PACKED;
-  if (packed && pairs->idx64) return GM_EINVAL;
-  if (pairs->mode == GM_PAIRS_SAMPLED && !packed) return GM_EINVAL;
-  if (loss->kind != GM_LOSS_QUOTIENT && loss->kind != GM_LOSS_STRESS) return GM_EINVAL;
-  if (loss->kind == GM_LOSS_QUOTIENT && !loss->inc_l1 && !loss->inc_l2) return GM_EINVAL;
+  if ((rc = check_loss(loss)) || (rc = check_fused_targets(pairs, targets))) return rc;
   if (pairs->P == 0) return GM_OK;
-  if (!acc || (!packed && !targets->data)) return GM_ENULL;
-  PairArgs a{};
-  fill_manifold(a, man);
-  a.kmode = K_FUSED;
-  a.ps = make_pairs(pairs);
+  if (!acc) return GM_ENULL;
+  PairArgs a = fused_args(man, pairs, targets, loss, scale_sp, acc, stream);
   a.sh.log2w = 0;
   while ((1 << a.sh.log2w) < W) ++a.sh.log2w;
   a.sh.mask = (unsigned)W - 1u;
@@ -326,51 +374,7 @@ int gm_pairs_loss_fused_sharded(const gm_manifold_t* man, const gm_row_shards_t*
     a.sh.x[r] = shards->x[r]; a.sh.g[r] = shards->grad[r];
   }
   a.xa = shards->x[0]; a.xb = shards->x[0]; a.ga = shards->grad[0]; a.gb = shards->grad[0]; a.out_d2 = out_d2;
-  a.tg = make_targets(targets);
-  if (packed) { a.tg.data = pairs->idx_j; a.ps.jmask = 0x00ffffffu; }
-  a.lc = make_loss(loss);
-  a.scale_sp = scale_sp;
-  a.acc = acc;
-  a.stream = (cudaStream_t)stream;
   return pair_dispatch(a);
-}
-
-int gm_product_loss(int32_t dtype, int32_t F, const void* const* d2_ptrs_host, const double* sp_host,
-                    const gm_pairs_t* pairs, const gm_targets_t* targets, const gm_loss_t* loss, int64_t P, double* acc,
-                    void* out_g, gm_stream_t stream) {
-  if (!d2_ptrs_host || !sp_host || !targets || !loss || !acc) return GM_ENULL;
-  if (F < 1 || F > 8 || P < 0) return GM_EINVAL;
-  if (dtype != GM_F32 && dtype != GM_F64) return GM_EINVAL;
-  if (targets->mode == GM_TGT_HOPS_PACKED) return GM_EINVAL;
-  PairSpec ps{};
-  if (targets->mode == GM_TGT_DENSE) {  // the pair enumeration gives the node ids that index the target matrix
-    int rc = validate_pairs(pairs);
-    if (rc) return rc;
-    if (pairs->mode == GM_PAIRS_ELEMENTWISE || pairs->P != P) return GM_EINVAL;
-    ps = make_pairs(pairs);
-  }
-  if (loss->kind != GM_LOSS_QUOTIENT && loss->kind != GM_LOSS_STRESS) return GM_EINVAL;
-  if (loss->kind == GM_LOSS_QUOTIENT && !loss->inc_l1 && !loss->inc_l2) return GM_EINVAL;
-  if (P == 0) return GM_OK;
-  FactorPtrs fp{};
-  for (int f = 0; f < F; ++f) {
-    if (!d2_ptrs_host[f]) return GM_ENULL;
-    fp.d2[f] = d2_ptrs_host[f];
-    fp.sp[f] = sp_host[f];
-  }
-  const int threads = 256;
-  long long blocks = (P + threads - 1) / threads;
-  if (blocks > 0x7fffffffLL) return GM_EINVAL;
-  TargetSpec tg = make_targets(targets);
-  LossCfg lc = make_loss(loss);
-  if (dtype == GM_F32)
-    product_loss_kernel<float><<<(unsigned)blocks, threads, 0, (cudaStream_t)stream>>>(F, fp, tg, ps, lc, P, acc,
-                                                                                       (float*)out_g);
-  else
-    product_loss_kernel<double><<<(unsigned)blocks, threads, 0, (cudaStream_t)stream>>>(F, fp, tg, ps, lc, P, acc,
-                                                                                        (double*)out_g);
-  note_launch();
-  return check_launch();
 }
 
 int gm_optim_step(const gm_manifold_t* man, const gm_optim_t* opt, void* x, void* grad, void* buf1, void* buf2,
@@ -379,19 +383,13 @@ int gm_optim_step(const gm_manifold_t* man, const gm_optim_t* opt, void* x, void
   if (rc) return rc;
   if (!opt) return GM_ENULL;
   if (N < 0) return GM_EINVAL;
-  if (opt->kind != GM_OPT_RSGD && opt->kind != GM_OPT_RADAM) return GM_EINVAL;
+  if (!optim_kind_ok(opt)) return GM_EINVAL;
   if (N == 0) return GM_OK;
   if (!x || !grad) return GM_ENULL;
-  if (opt->kind == GM_OPT_RADAM && (!buf1 || !buf2 || opt->step < 1)) return GM_EINVAL;
-  if (opt->kind == GM_OPT_RSGD && opt->has_momentum && !buf1) return GM_ENULL;
-  PointArgs a{};
-  a.kind = man->kind; a.dtype = man->dtype; a.n = man->n; a.p = man->p; a.flags = man->flags;
-  a.wmin = man->wmin; a.wmax = man->wmax; a.c_dev = man->c_dev;
-  a.op = -1;
-  a.oc = make_optim_cfg(opt);
-  a.grassmann_retr_qr = opt->grassmann_retr_qr;
-  a.x = x; a.u = grad; a.buf1 = buf1; a.buf2 = (opt->kind == GM_OPT_RADAM) ? buf2 : nullptr;
-  if (opt->kind == GM_OPT_RSGD && !opt->has_momentum) a.buf1 = nullptr;
+  rc = check_optim(opt, buf1, buf2);
+  if (rc) return rc;
+  PointArgs a = point_args(man, opt, buf1, buf2);
+  a.x = x; a.u = grad;
   a.N = N;
   a.stream = (cudaStream_t)stream;
   return point_dispatch(a);
@@ -408,35 +406,27 @@ int gm_train_epoch(const gm_manifold_t* man, const gm_optim_t* opt, void* x, voi
   if (man->kind == GM_UNIVERSAL) return GM_EUNSUPPORTED;  // the curvature gradient needs the autograd-side chain rule
   if (N <= 0 || n_perm < 0 || batch_nodes < 2 || max_steps < 0) return GM_EINVAL;
   if (targets->mode != GM_TGT_DENSE || !targets->data) return GM_EINVAL;
-  if (opt->kind != GM_OPT_RSGD && opt->kind != GM_OPT_RADAM) return GM_EINVAL;
-  if (loss->kind != GM_LOSS_QUOTIENT && loss->kind != GM_LOSS_STRESS) return GM_EINVAL;
-  if (loss->kind == GM_LOSS_QUOTIENT && !loss->inc_l1 && !loss->inc_l2) return GM_EINVAL;
+  if (!optim_kind_ok(opt)) return GM_EINVAL;
+  rc = check_loss(loss);
+  if (rc) return rc;
   if (!x || !grad || !perm || !acc) return GM_ENULL;
-  if (opt->kind == GM_OPT_RADAM && (!buf1 || !buf2 || opt->step < 1)) return GM_EINVAL;
-  if (opt->kind == GM_OPT_RSGD && opt->has_momentum && !buf1) return GM_ENULL;
+  rc = check_optim(opt, buf1, buf2);
+  if (rc) return rc;
   const size_t grad_bytes = (size_t)N * point_elems(man) * (man->dtype == GM_F32 ? 4 : 8);
-  const size_t idx_bytes = perm_is_int64 ? 8 : 4;
   cudaStream_t st = (cudaStream_t)stream;
   gm_optim_t o = *opt;
-  int64_t k = 0;
-  for (int64_t i = 0; i < n_perm; i += batch_nodes, ++k) {
-    const int64_t b = (n_perm - i < batch_nodes) ? (n_perm - i) : batch_nodes;
-    if (b < drop_last_n || b < 2) break;
-    if (k >= max_steps) return GM_EINVAL;
+  return for_each_node_batch(perm, perm_is_int64, n_perm, batch_nodes, drop_last_n, max_steps, n_steps,
+                             [&](int64_t k, const gm_pairs_t& pr) -> int {
     cudaError_t e = cudaMemsetAsync(grad, 0, grad_bytes, st);
     if (e != cudaSuccess) return (int)e;
-    gm_pairs_t pr{};
-    pr.mode = GM_PAIRS_TRIU; pr.idx64 = perm_is_int64; pr.P = b * (b - 1) / 2; pr.B = b;
-    pr.nodes = (const char*)perm + (size_t)i * idx_bytes; pr.k0 = 0;
-    rc = gm_pairs_loss_fused(man, x, &pr, targets, loss, scale_sp, nullptr, acc + 2 * k, grad, stream);
+    int rc = gm_pairs_loss_fused(man, x, &pr, targets, loss, scale_sp, nullptr, acc + 2 * k, grad, stream);
     if (rc) return rc;
     rc = gm_optim_step(man, &o, x, grad, buf1, buf2, N, stream);
     if (rc) return rc;
     o.step += 1;       // RAdam: state['step'] += 1 (radam.py:98)
     o.first_step = 0;  // RSGD momentum buffer exists from now on
-  }
-  *n_steps = k;
-  return GM_OK;
+    return GM_OK;
+  });
 }
 
 // Can the fused product kernel (gm_product.cuh) take this factor list?  At most one SPD factor, the rest Lorentz /
@@ -466,15 +456,9 @@ int gm_pairs_product_fused(int32_t F, const gm_manifold_t* mans, void* const* x,
   if (!product_fusable(F, mans)) return GM_EUNSUPPORTED;
   int rc = validate_pairs(pairs);
   if (rc) return rc;
-  if (pairs->mode == GM_PAIRS_ELEMENTWISE) return GM_EINVAL;
-  if (targets->mode < GM_TGT_VECTOR || targets->mode > GM_TGT_HOPS_PACKED) return GM_EINVAL;
-  const bool packed = targets->mode == GM_TGT_HOPS_PACKED;
-  if (packed && ((pairs->mode != GM_PAIRS_LIST && pairs->mode != GM_PAIRS_SAMPLED) || pairs->idx64)) return GM_EINVAL;
-  if (pairs->mode == GM_PAIRS_SAMPLED && !packed) return GM_EINVAL;
-  if (loss->kind != GM_LOSS_QUOTIENT && loss->kind != GM_LOSS_STRESS) return GM_EINVAL;
-  if (loss->kind == GM_LOSS_QUOTIENT && !loss->inc_l1 && !loss->inc_l2) return GM_EINVAL;
+  if ((rc = check_loss(loss)) || (rc = check_fused_targets(pairs, targets))) return rc;
   if (pairs->P == 0) return GM_OK;
-  if (!acc || (!packed && !targets->data)) return GM_ENULL;
+  if (!acc) return GM_ENULL;
   ProductExtra px{};
   px.F = F; px.lead_slot = -1; px.nvec = 0;
   for (int f = 0; f < F; ++f) {
@@ -483,22 +467,13 @@ int gm_pairs_product_fused(int32_t F, const gm_manifold_t* mans, void* const* x,
     VecExtra& v = px.v[px.nvec++];
     v.kind = mans[f].kind; v.n = mans[f].n; v.slot = f; v.x = x[f]; v.g = grad[f]; v.sp = sp[f];
   }
-  PairArgs a{};
-  if (px.lead_slot >= 0) {
-    fill_manifold(a, &mans[px.lead_slot]);
-    a.xa = a.xb = x[px.lead_slot];
-    a.ga = a.gb = grad[px.lead_slot];
-    a.scale_sp = sp[px.lead_slot];
-  } else {
-    fill_manifold(a, &mans[0]);  // dtype; the factors themselves travel in px
+  const int lead = px.lead_slot;
+  // without an SPD factor, mans[0] gives the dtype and the factors themselves travel in px
+  PairArgs a = fused_args(&mans[lead >= 0 ? lead : 0], pairs, targets, loss, lead >= 0 ? sp[lead] : 0.0, acc, stream);
+  if (lead >= 0) {
+    a.xa = a.xb = x[lead];
+    a.ga = a.gb = grad[lead];
   }
-  a.kmode = K_FUSED;
-  a.ps = make_pairs(pairs);
-  a.tg = make_targets(targets);
-  if (packed) { a.tg.data = pairs->idx_j; a.ps.jmask = 0x00ffffffu; }
-  a.lc = make_loss(loss);
-  a.acc = acc;
-  a.stream = (cudaStream_t)stream;
   a.px = &px;
   return pair_dispatch(a);
 }
@@ -518,25 +493,16 @@ int gm_train_epoch_product(int32_t F, const gm_manifold_t* mans, const gm_optim_
     if (mans[f].kind == GM_UNIVERSAL) return GM_EUNSUPPORTED;
     if (mans[f].dtype != mans[0].dtype) return GM_EINVAL;
     if (!x[f] || !grad[f] || !d2_ws[f]) return GM_ENULL;
-    if (opts[f].kind != GM_OPT_RSGD && opts[f].kind != GM_OPT_RADAM) return GM_EINVAL;
-    if (opts[f].kind == GM_OPT_RADAM && (!buf1[f] || !buf2[f] || opts[f].step < 1)) return GM_EINVAL;
-    if (opts[f].kind == GM_OPT_RSGD && opts[f].has_momentum && !buf1[f]) return GM_ENULL;
+    rc = check_optim(&opts[f], buf1[f], buf2[f]);
+    if (rc) return rc;
   }
   const size_t s_bytes = mans[0].dtype == GM_F32 ? 4 : 8;
-  const size_t idx_bytes = perm_is_int64 ? 8 : 4;
   cudaStream_t st = (cudaStream_t)stream;
   gm_optim_t o[8];
   for (int f = 0; f < F; ++f) o[f] = opts[f];
-  const char* fuse_env = getenv("GM_PRODUCT_FUSED");  // "0": keep the unfused 2 F + 1 pair launches per step (A/B, tests)
-  const bool fused = !(fuse_env && fuse_env[0] == '0') && product_fusable(F, mans);
-  int64_t k = 0;
-  for (int64_t i = 0; i < n_perm; i += batch_nodes, ++k) {
-    const int64_t b = (n_perm - i < batch_nodes) ? (n_perm - i) : batch_nodes;
-    if (b < drop_last_n || b < 2) break;
-    if (k >= max_steps) return GM_EINVAL;
-    gm_pairs_t pr{};
-    pr.mode = GM_PAIRS_TRIU; pr.idx64 = perm_is_int64; pr.P = b * (b - 1) / 2; pr.B = b;
-    pr.nodes = (const char*)perm + (size_t)i * idx_bytes; pr.k0 = 0;
+  const bool fused = product_fusable(F, mans);
+  return for_each_node_batch(perm, perm_is_int64, n_perm, batch_nodes, drop_last_n, max_steps, n_steps,
+                             [&](int64_t k, const gm_pairs_t& pr) -> int {
     for (int f = 0; f < F; ++f) {
       cudaError_t e = cudaMemsetAsync(grad[f], 0, (size_t)N * point_elems(&mans[f]) * s_bytes, st);
       if (e != cudaSuccess) return (int)e;
@@ -558,9 +524,8 @@ int gm_train_epoch_product(int32_t F, const gm_manifold_t* mans, const gm_optim_
       o[f].step += 1;
       o[f].first_step = 0;
     }
-  }
-  *n_steps = k;
-  return GM_OK;
+    return GM_OK;
+  });
 }
 
 int gm_peer_alloc(size_t bytes, void** ptr) {
@@ -596,35 +561,12 @@ int gm_optim_step_peer(const gm_manifold_t* man, const gm_optim_t* opt, const gm
   if (N_owned <= 0 || peers->row_lo < 0 || peers->epoch == 0) return GM_EINVAL;  // every rank must launch: no empty shards
   if (peers->world < 1 || peers->world > GM_MAX_PEERS || peers->rank < 0 || peers->rank >= peers->world) return GM_EINVAL;
   if (peers->n_acc < 0 || peers->n_acc > 64) return GM_EINVAL;
-  if (opt->kind != GM_OPT_RSGD && opt->kind != GM_OPT_RADAM) return GM_EINVAL;
-  if (opt->kind == GM_OPT_RADAM && (!buf1 || !buf2 || opt->step < 1)) return GM_EINVAL;
-  if (opt->kind == GM_OPT_RSGD && opt->has_momentum && !buf1) return GM_ENULL;
-  PeerTable pt{};
-  pt.world = peers->world; pt.rank = peers->rank; pt.row_lo = peers->row_lo; pt.epoch = peers->epoch;
-  for (int r = 0; r < peers->world; ++r) {
-    if (!peers->x[r] || !peers->grad[r] || !peers->flags[r]) return GM_ENULL;
-    if (peers->n_acc > 0 && !peers->acc[r]) return GM_ENULL;
-    pt.x[r] = peers->x[r]; pt.g[r] = peers->grad[r];
-    pt.flags[r] = (unsigned long long*)peers->flags[r];
-    pt.acc[r] = (const double*)peers->acc[r];
-  }
-  if (peers->n_acc > 0 && !peers->acc_out) return GM_ENULL;
-  pt.acc_out = (double*)peers->acc_out; pt.n_acc = peers->n_acc;
-  pt.gsum = peers->gsum;
-  {
-    static const long long timeout_s = [] { const char* e = getenv("GM_PEER_TIMEOUT_S"); return e ? atoll(e) : 300LL; }();
-    static const int chunks = [] { const char* e = getenv("GM_PEER_CHUNKS"); return e ? atoi(e) : 4; }();
-    pt.timeout_ns = timeout_s > 0 ? (unsigned long long)timeout_s * 1000000000ull : 0ull;
-    pt.chunks = chunks;
-  }
-  PointArgs a{};
-  a.kind = man->kind; a.dtype = man->dtype; a.n = man->n; a.p = man->p; a.flags = man->flags;
-  a.wmin = man->wmin; a.wmax = man->wmax; a.c_dev = man->c_dev;
-  a.op = -1;
-  a.oc = make_optim_cfg(opt);
-  a.grassmann_retr_qr = opt->grassmann_retr_qr;
-  a.buf1 = buf1; a.buf2 = (opt->kind == GM_OPT_RADAM) ? buf2 : nullptr;
-  if (opt->kind == GM_OPT_RSGD && !opt->has_momentum) a.buf1 = nullptr;
+  rc = check_optim(opt, buf1, buf2);
+  if (rc) return rc;
+  PeerTable pt;
+  rc = peer_table(peers, -1, pt);
+  if (rc) return rc;
+  PointArgs a = point_args(man, opt, buf1, buf2);
   a.N = N_owned;
   a.stream = (cudaStream_t)stream;
   a.peer = &pt;
@@ -635,20 +577,9 @@ int gm_peer_barrier(const gm_peers_t* peers, int32_t phase, gm_stream_t stream) 
   if (!peers) return GM_ENULL;
   if (peers->world < 1 || peers->world > GM_MAX_PEERS || peers->rank < 0 || peers->rank >= peers->world) return GM_EINVAL;
   if (phase < 0 || phase > 1 || peers->epoch == 0 || peers->n_acc < 0 || peers->n_acc > 64) return GM_EINVAL;
-  PeerTable pt{};
-  pt.world = peers->world; pt.rank = peers->rank; pt.epoch = peers->epoch;
-  for (int r = 0; r < peers->world; ++r) {
-    if (!peers->flags[r]) return GM_ENULL;
-    if (phase == 0 && peers->n_acc > 0 && !peers->acc[r]) return GM_ENULL;
-    pt.flags[r] = (unsigned long long*)peers->flags[r];
-    pt.acc[r] = (const double*)peers->acc[r];
-  }
-  if (phase == 0 && peers->n_acc > 0 && !peers->acc_out) return GM_ENULL;
-  pt.acc_out = (double*)peers->acc_out; pt.n_acc = phase == 0 ? peers->n_acc : 0;
-  {
-    static const long long timeout_s = [] { const char* e = getenv("GM_PEER_TIMEOUT_S"); return e ? atoll(e) : 300LL; }();
-    pt.timeout_ns = timeout_s > 0 ? (unsigned long long)timeout_s * 1000000000ull : 0ull;
-  }
+  PeerTable pt;
+  int rc = peer_table(peers, phase, pt);
+  if (rc) return rc;
   return launch_peer_barrier(pt, phase, (cudaStream_t)stream);
 }
 
@@ -663,11 +594,8 @@ int gm_point_op(const gm_manifold_t* man, int32_t op, const void* x, const void*
   const bool needs_u = op != GM_OP_PROJX && op != GM_OP_SPD_SQRTM;
   const bool needs_v = op == GM_OP_INNER || op == GM_OP_TRANSP;
   if ((needs_u && !u) || (needs_v && !v)) return GM_ENULL;
-  PointArgs a{};
-  a.kind = man->kind; a.dtype = man->dtype; a.n = man->n; a.p = man->p; a.flags = man->flags;
-  a.wmin = man->wmin; a.wmax = man->wmax; a.c_dev = man->c_dev;
+  PointArgs a = point_args(man, nullptr, nullptr, nullptr);
   a.op = op;
-  a.grassmann_retr_qr = 0;
   if (op == GM_OP_RETR_QR) { a.op = GM_OP_RETR; a.grassmann_retr_qr = 1; }
   a.x = const_cast<void*>(x); a.u = u; a.v = v; a.out = out;
   a.N = N;

@@ -81,6 +81,7 @@ inline LossCfg make_loss(const gm_loss_t* l) {
   return c;
 }
 int validate_pairs(const gm_pairs_t* p);
+int check_loss(const gm_loss_t* loss);
 
 // factor distance vectors of a product manifold and their softplus(scale) weights (modules.py:84-88)
 struct FactorPtrs {
@@ -126,6 +127,37 @@ struct PairArgs {
   const ProductExtra* px;  // K_FUSED only: non-null = product-manifold launch (acc has 1 + F slots)
   ShardTab sh;             // row-sharded tables (xa / xb / ga / gb ignored) when sh.log2w >= 0
 };
+
+// The per-mode kernel arguments of a pair launch: the buffers a mode does not use are passed as NULL / 0.
+template <typename T, int KMODE>
+struct ModeArgs {
+  static constexpr int kmode = KMODE;
+  const T* gout;
+  T coef;
+  T* ga;
+  T* gb;
+  T* out_d2;
+  T scale_sp;
+  double* acc;
+  double* c_grad;
+  explicit ModeArgs(const PairArgs& a)
+      : gout(KMODE == K_BWD ? (const T*)a.gout : nullptr), coef(KMODE == K_BWD ? (T)a.coef : (T)0),
+        ga(KMODE == K_FWD ? nullptr : (T*)a.ga), gb(KMODE == K_FWD ? nullptr : (T*)a.gb),
+        out_d2(KMODE == K_BWD ? nullptr : (T*)a.out_d2), scale_sp(KMODE == K_FUSED ? (T)a.scale_sp : (T)0),
+        acc(KMODE == K_FUSED ? a.acc : nullptr), c_grad(KMODE == K_FWD ? nullptr : a.c_grad) {}
+};
+
+// launch(ModeArgs<T, a.kmode>) for a one-pair-per-thread kernel, counted
+template <typename T, class Launch>
+int launch_by_mode(const PairArgs& a, Launch&& launch) {
+  switch (a.kmode) {
+    case K_FWD: launch(ModeArgs<T, K_FWD>(a)); break;
+    case K_BWD: launch(ModeArgs<T, K_BWD>(a)); break;
+    default: launch(ModeArgs<T, K_FUSED>(a));
+  }
+  note_launch();
+  return check_launch();
+}
 
 // ---- pair enumeration --------------------------------------------------------
 __device__ __forceinline__ long long load_index(const void* p, long long k, int idx64) {
@@ -173,21 +205,7 @@ __device__ __forceinline__ unsigned sampled_j(const PairSpec& ps, long long k, l
 }
 // One random byte out of a multi-GB table per pair: streaming (evict-first) so that it does not push the gradient and
 // point tables out of L2.
-#ifndef GM_HOP_LOAD
-#define GM_HOP_LOAD 0
-#endif
-__device__ __forceinline__ unsigned load_hop(const unsigned char* p) {
-#if GM_HOP_LOAD == 0
-  return (unsigned)__ldcs(p);
-#elif GM_HOP_LOAD == 1
-  return (unsigned)__ldg(p);
-#elif GM_HOP_LOAD == 2
-  return (unsigned)*p;
-#else  // aligned 32-bit load of the word that holds the byte
-  const unsigned w = __ldg(reinterpret_cast<const unsigned*>(reinterpret_cast<size_t>(p) & ~(size_t)3));
-  return (w >> (8 * (unsigned)(reinterpret_cast<size_t>(p) & 3))) & 0xFFu;
-#endif
-}
+__device__ __forceinline__ unsigned load_hop(const unsigned char* p) { return (unsigned)__ldcs(p); }
 __device__ __forceinline__ unsigned sampled_word(const PairSpec& ps, long long k, long long& ra) {
   const unsigned char* hp;
   const unsigned j = sampled_j(ps, k, ra, hp);

@@ -38,6 +38,40 @@ pairs_metrics_kernel(int F, FactorPtrs fp, PairSpec ps, TargetSpec tg, int squar
 }
 
 // ---------------------------------------------------------------------------
+// product-manifold loss over F distance vectors
+// ---------------------------------------------------------------------------
+template <typename T>
+__global__ void __launch_bounds__(256)
+product_loss_kernel(int F, FactorPtrs fp, TargetSpec tg, PairSpec ps, LossCfg lc, long long P,
+                    double* __restrict__ acc, T* __restrict__ out_g) {
+  __shared__ double red[8];
+  long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  bool active = k < P;
+  double lv = 0.0;
+  double gd[8];
+  for (int f = 0; f < 8; ++f) gd[f] = 0.0;
+  if (active) {
+    // sum() of a Python list starts from int 0 and adds left to right (modules.py:84-88)
+    T m = (T)0;
+    T d2[8];
+    for (int f = 0; f < F; ++f) {
+      d2[f] = ((const T*)fp.d2[f])[k];
+      T term = (T)fp.sp[f] * d2[f];
+      m = (f == 0) ? term : m + term;
+    }
+    long long ra = 0, rb = 0;
+    if (tg.mode == GM_TGT_DENSE) decode_pair(ps, k, ra, rb);  // node ids index the dense target matrix
+    T g = fetch_target<T>(tg, k, ra, rb);
+    T dm;
+    lv = (double)loss_term<T>(lc, g, m, dm);
+    if (out_g) out_g[k] = dm;
+    for (int f = 0; f < F; ++f) gd[f] = (double)dm * (double)d2[f];
+  }
+  block_accumulate(lv, acc, red);
+  for (int f = 0; f < F; ++f) block_accumulate(gd[f], acc + 1 + f, red);
+}
+
+// ---------------------------------------------------------------------------
 // stochastic-neighbour KL objective
 // ---------------------------------------------------------------------------
 struct SneCfg {
@@ -201,6 +235,44 @@ int gm_pairs_metrics(int32_t dtype, int32_t F, const void* const* d2_ptrs_host, 
     pairs_metrics_kernel<float><<<blocks, threads, 0, (cudaStream_t)stream>>>(F, fp, ps, tg, squared_inputs, acc);
   else
     pairs_metrics_kernel<double><<<blocks, threads, 0, (cudaStream_t)stream>>>(F, fp, ps, tg, squared_inputs, acc);
+  note_launch();
+  return check_launch();
+}
+
+int gm_product_loss(int32_t dtype, int32_t F, const void* const* d2_ptrs_host, const double* sp_host,
+                    const gm_pairs_t* pairs, const gm_targets_t* targets, const gm_loss_t* loss, int64_t P, double* acc,
+                    void* out_g, gm_stream_t stream) {
+  if (!d2_ptrs_host || !sp_host || !targets || !loss || !acc) return GM_ENULL;
+  if (F < 1 || F > 8 || P < 0) return GM_EINVAL;
+  if (dtype != GM_F32 && dtype != GM_F64) return GM_EINVAL;
+  if (targets->mode == GM_TGT_HOPS_PACKED) return GM_EINVAL;
+  PairSpec ps{};
+  if (targets->mode == GM_TGT_DENSE) {  // the pair enumeration gives the node ids that index the target matrix
+    int rc = validate_pairs(pairs);
+    if (rc) return rc;
+    if (pairs->mode == GM_PAIRS_ELEMENTWISE || pairs->P != P) return GM_EINVAL;
+    ps = make_pairs(pairs);
+  }
+  int rc = check_loss(loss);
+  if (rc) return rc;
+  if (P == 0) return GM_OK;
+  FactorPtrs fp{};
+  for (int f = 0; f < F; ++f) {
+    if (!d2_ptrs_host[f]) return GM_ENULL;
+    fp.d2[f] = d2_ptrs_host[f];
+    fp.sp[f] = sp_host[f];
+  }
+  const int threads = 256;
+  long long blocks = (P + threads - 1) / threads;
+  if (blocks > 0x7fffffffLL) return GM_EINVAL;
+  TargetSpec tg = make_targets(targets);
+  LossCfg lc = make_loss(loss);
+  if (dtype == GM_F32)
+    product_loss_kernel<float><<<(unsigned)blocks, threads, 0, (cudaStream_t)stream>>>(F, fp, tg, ps, lc, P, acc,
+                                                                                       (float*)out_g);
+  else
+    product_loss_kernel<double><<<(unsigned)blocks, threads, 0, (cudaStream_t)stream>>>(F, fp, tg, ps, lc, P, acc,
+                                                                                        (double*)out_g);
   note_launch();
   return check_launch();
 }

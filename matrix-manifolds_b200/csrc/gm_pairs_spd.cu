@@ -491,21 +491,16 @@ static int launch_op(const Op& op, const PairArgs& a) {
   dim3 grid((unsigned)blocks), block(threads);
   const T* xa = (const T*)a.xa;
   const T* xb = (const T*)a.xb;
-#ifndef GM_MINB_F32
-#define GM_MINB_F32 4
-#endif
-#ifndef GM_PF_DEPTH
-#define GM_PF_DEPTH 1
-#endif
-  constexpr int MINB = sizeof(T) == 4 ? GM_MINB_F32 : 2;
-  // rows stay in flight for two iterations when MINB CTAs of three staging slots still fit one SM's shared memory
-  constexpr int DEPTH = (RowStage<T, Op::E, GM_PF_DEPTH + 1>::BYTES + 3 * 1024) * MINB <= 224 * 1024 ? GM_PF_DEPTH : 1;
+  constexpr int MINB = sizeof(T) == 4 ? 4 : 2;  // resident CTAs per SM the streaming kernel is built for
+  constexpr int DEPTH = 1;                      // a pair's rows are in flight for one iteration of its loop
   using Stage = RowStage<T, Op::E, DEPTH + 1>;
   if (a.kmode != K_FWD && a.ps.mode != GM_PAIRS_ELEMENTWISE && RowStage<T, Op::E, 2>::BYTES <= 64 * 1024) {
     int dev = 0, sms = 0, occ = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    auto launch_stream = [&](auto kern, auto spec_kern, const T* gout, T coef, T* out_d2, T scale, double* acc) -> int {
+    auto launch_stream = [&](auto m) -> int {
+      constexpr int KMODE = decltype(m)::kmode;
+      auto kern = spd_pair_stream_kernel<Op, T, KMODE, MINB, DEPTH>;
       cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Stage::BYTES);
       cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, Stage::BYTES);
       if (occ < 1) occ = 1;
@@ -518,47 +513,29 @@ static int launch_op(const Op& op, const PairArgs& a) {
       ps.seg_len = (ps.P + ps.nseg - 1) / ps.nseg;
       long long chunk = ((ps.seg_len + warps - 1) / warps + 31) / 32 * 32;
       if (chunk * ps.nseg > 0x7fffffffLL) return GM_EINVAL;
-#ifndef GM_NO_SPEC
-      if constexpr (GM_N == 4 && sizeof(T) == 4 && Op::kCanPrep) {  // the window-ordered config 5 step: see SPEC
-        if (spec_kern && ps.nseg > 1 && !ps.idx64 && a.tg.mode == GM_TGT_HOPS_PACKED && a.sh.log2w < 0) {
-          cudaFuncSetAttribute(spec_kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Stage::BYTES);
-          spec_kern<<<(unsigned)nb, threads, Stage::BYTES, a.stream>>>(op, ps, xa, xb, gout, coef, (T*)a.ga, (T*)a.gb,
-                                                                    out_d2, a.tg, a.lc, scale, acc, chunk, a.sh);
+      if constexpr (KMODE == K_FUSED && GM_N == 4 && sizeof(T) == 4 && Op::kCanPrep) {  // the window-ordered config 5 step: see SPEC
+        if (ps.nseg > 1 && !ps.idx64 && a.tg.mode == GM_TGT_HOPS_PACKED && a.sh.log2w < 0) {
+          auto spec = spd_pair_stream_kernel<Op, T, K_FUSED, MINB, DEPTH, 1>;
+          cudaFuncSetAttribute(spec, cudaFuncAttributeMaxDynamicSharedMemorySize, Stage::BYTES);
+          spec<<<(unsigned)nb, threads, Stage::BYTES, a.stream>>>(op, ps, xa, xb, m.gout, m.coef, m.ga, m.gb, m.out_d2,
+                                                                   a.tg, a.lc, m.scale_sp, m.acc, chunk, a.sh);
           note_launch();
           return check_launch();
         }
       }
-#endif
-      kern<<<(unsigned)nb, threads, Stage::BYTES, a.stream>>>(op, ps, xa, xb, gout, coef, (T*)a.ga, (T*)a.gb, out_d2,
-                                                             a.tg, a.lc, scale, acc, chunk, a.sh);
+      kern<<<(unsigned)nb, threads, Stage::BYTES, a.stream>>>(op, ps, xa, xb, m.gout, m.coef, m.ga, m.gb, m.out_d2, a.tg,
+                                                             a.lc, m.scale_sp, m.acc, chunk, a.sh);
       note_launch();
       return check_launch();
     };
-    using kern_t = decltype(&spd_pair_stream_kernel<Op, T, K_FUSED, MINB, DEPTH>);
-    if (a.kmode == K_BWD)
-      return launch_stream(spd_pair_stream_kernel<Op, T, K_BWD, MINB, DEPTH>, (kern_t) nullptr, (const T*)a.gout,
-                           (T)a.coef, nullptr, (T)0, nullptr);
-    kern_t spec = nullptr;
-    if constexpr (GM_N == 4 && sizeof(T) == 4 && Op::kCanPrep) spec = spd_pair_stream_kernel<Op, T, K_FUSED, MINB, DEPTH, 1>;
-    return launch_stream(spd_pair_stream_kernel<Op, T, K_FUSED, MINB, DEPTH>, spec, nullptr, (T)0, (T*)a.out_d2,
-                         (T)a.scale_sp, a.acc);
+    if (a.kmode == K_BWD) return launch_stream(ModeArgs<T, K_BWD>(a));
+    return launch_stream(ModeArgs<T, K_FUSED>(a));
   }
   if (a.sh.log2w >= 0) return GM_EUNSUPPORTED;  // row-sharded tables: the streaming (training) kernels only
-  switch (a.kmode) {
-    case K_FWD:
-      spd_pair_kernel<Op, T, K_FWD><<<grid, block, 0, a.stream>>>(
-          op, a.ps, xa, xb, nullptr, (T)0, nullptr, nullptr, (T*)a.out_d2, a.tg, a.lc, (T)0, nullptr);
-      break;
-    case K_BWD:
-      spd_pair_kernel<Op, T, K_BWD><<<grid, block, 0, a.stream>>>(
-          op, a.ps, xa, xb, (const T*)a.gout, (T)a.coef, (T*)a.ga, (T*)a.gb, nullptr, a.tg, a.lc, (T)0, nullptr);
-      break;
-    default:
-      spd_pair_kernel<Op, T, K_FUSED><<<grid, block, 0, a.stream>>>(
-          op, a.ps, xa, xb, nullptr, (T)0, (T*)a.ga, (T*)a.gb, (T*)a.out_d2, a.tg, a.lc, (T)a.scale_sp, a.acc);
-  }
-  note_launch();
-  return check_launch();
+  return launch_by_mode<T>(a, [&](auto m) {
+    spd_pair_kernel<Op, T, decltype(m)::kmode><<<grid, block, 0, a.stream>>>(
+        op, a.ps, xa, xb, m.gout, m.coef, m.ga, m.gb, m.out_d2, a.tg, a.lc, m.scale_sp, m.acc);
+  });
 }
 
 template <typename T>

@@ -150,29 +150,30 @@ grassmann_pair_kernel(GrassmannCore<T, P, FAST> op, int n, PairSpec ps, const T*
   }
 }
 
-#define GM_LAUNCH3(KERNEL, OP, ...)                                                                               \
-  switch (a.kmode) {                                                                                             \
-    case K_FWD:                                                                                                  \
-      KERNEL<__VA_ARGS__, K_FWD><<<grid, block, 0, a.stream>>>(OP, a.n, a.ps, xa, xb, nullptr, (T)0, nullptr,     \
-                                                               nullptr, (T*)a.out_d2, a.tg, a.lc, (T)0, nullptr, \
-                                                               nullptr);                                          \
-      break;                                                                                                     \
-    case K_BWD:                                                                                                  \
-      KERNEL<__VA_ARGS__, K_BWD><<<grid, block, 0, a.stream>>>(OP, a.n, a.ps, xa, xb, (const T*)a.gout,           \
-                                                               (T)a.coef, (T*)a.ga, (T*)a.gb, nullptr, a.tg,      \
-                                                               a.lc, (T)0, nullptr, a.c_grad);                    \
-      break;                                                                                                     \
-    default:                                                                                                     \
-      KERNEL<__VA_ARGS__, K_FUSED><<<grid, block, 0, a.stream>>>(OP, a.n, a.ps, xa, xb, nullptr, (T)0,            \
-                                                                 (T*)a.ga, (T*)a.gb, (T*)a.out_d2, a.tg, a.lc,    \
-                                                                 (T)a.scale_sp, a.acc, a.c_grad);                 \
-  }
-
 template <typename T>
 static T one_minus_eps2() {
   // `1 - EPS[dtype]**2` is evaluated by Python in double and then cast by torch's
   // clamp_ to the tensor dtype (sphere.py:70, grassmann.py:94)
   return (T)(1.0 - 1e-8 * 1e-8);
+}
+
+template <typename T, int KIND>
+static int launch_vec(const PairArgs& a, dim3 grid, dim3 block, VecMan<T, KIND> op) {
+  return launch_by_mode<T>(a, [&](auto m) {
+    vec_pair_kernel<T, KIND, decltype(m)::kmode><<<grid, block, 0, a.stream>>>(
+        op, a.n, a.ps, (const T*)a.xa, (const T*)a.xb, m.gout, m.coef, m.ga, m.gb, m.out_d2, a.tg, a.lc, m.scale_sp,
+        m.acc, m.c_grad);
+  });
+}
+
+template <typename T, int P, bool FAST>
+static int launch_grassmann(const PairArgs& a, dim3 grid, dim3 block) {
+  GrassmannCore<T, P, FAST> op{one_minus_eps2<T>()};
+  return launch_by_mode<T>(a, [&](auto m) {
+    grassmann_pair_kernel<T, P, FAST, decltype(m)::kmode><<<grid, block, 0, a.stream>>>(
+        op, a.n, a.ps, (const T*)a.xa, (const T*)a.xb, m.gout, m.coef, m.ga, m.gb, m.out_d2, a.tg, a.lc, m.scale_sp,
+        m.acc, m.c_grad);
+  });
 }
 
 template <typename T>
@@ -182,49 +183,25 @@ static int vec_launch_typed(const PairArgs& a) {
   long long blocks = (a.ps.P + threads - 1) / threads;
   if (blocks > 0x7fffffffLL) return GM_EINVAL;
   dim3 grid((unsigned)blocks), block(threads);
-  const T* xa = (const T*)a.xa;
-  const T* xb = (const T*)a.xb;
   const T eps = (T)1e-8;
-  if (a.kind == GM_LORENTZ) {
-    VecMan<T, VEC_LORENTZ> op{eps, one_minus_eps2<T>(), nullptr};
-    GM_LAUNCH3(vec_pair_kernel, op, T, VEC_LORENTZ)
-  } else if (a.kind == GM_SPHERE) {
-    VecMan<T, VEC_SPHERE> op{eps, one_minus_eps2<T>(), nullptr};
-    GM_LAUNCH3(vec_pair_kernel, op, T, VEC_SPHERE)
-  } else if (a.kind == GM_EUCLIDEAN) {
-    VecMan<T, VEC_EUCLIDEAN> op{eps, one_minus_eps2<T>(), nullptr};
-    GM_LAUNCH3(vec_pair_kernel, op, T, VEC_EUCLIDEAN)
-  } else if (a.kind == GM_UNIVERSAL) {
-    VecMan<T, VEC_UNIVERSAL> op{(T)a.wmin, one_minus_eps2<T>(), (const T*)a.c_dev};  // value floor: wmin
-    GM_LAUNCH3(vec_pair_kernel, op, T, VEC_UNIVERSAL)
-  } else if (a.kind == GM_GRASSMANN) {
-    const bool fast = (a.flags & GM_FAST_SVD) != 0;
-    if (a.p == 2 && fast) {
-      GrassmannCore<T, 2, true> op{one_minus_eps2<T>()};
-      GM_LAUNCH3(grassmann_pair_kernel, op, T, 2, true)
-    } else if (a.p == 1) {
-      GrassmannCore<T, 1, false> op{one_minus_eps2<T>()};
-      GM_LAUNCH3(grassmann_pair_kernel, op, T, 1, false)
-    } else if (a.p == 2) {
-      GrassmannCore<T, 2, false> op{one_minus_eps2<T>()};
-      GM_LAUNCH3(grassmann_pair_kernel, op, T, 2, false)
-    } else if (a.p == 3) {
-      GrassmannCore<T, 3, false> op{one_minus_eps2<T>()};
-      GM_LAUNCH3(grassmann_pair_kernel, op, T, 3, false)
-    } else if (a.p == 4) {
-      GrassmannCore<T, 4, false> op{one_minus_eps2<T>()};
-      GM_LAUNCH3(grassmann_pair_kernel, op, T, 4, false)
-    } else if (a.p == 5) {
-      GrassmannCore<T, 5, false> op{one_minus_eps2<T>()};
-      GM_LAUNCH3(grassmann_pair_kernel, op, T, 5, false)
-    } else {
-      return GM_EUNSUPPORTED;
-    }
-  } else {
-    return GM_EINVAL;
+  switch (a.kind) {
+    case GM_LORENTZ: return launch_vec(a, grid, block, VecMan<T, VEC_LORENTZ>{eps, one_minus_eps2<T>(), nullptr});
+    case GM_SPHERE: return launch_vec(a, grid, block, VecMan<T, VEC_SPHERE>{eps, one_minus_eps2<T>(), nullptr});
+    case GM_EUCLIDEAN: return launch_vec(a, grid, block, VecMan<T, VEC_EUCLIDEAN>{eps, one_minus_eps2<T>(), nullptr});
+    case GM_UNIVERSAL:  // value floor: wmin
+      return launch_vec(a, grid, block, VecMan<T, VEC_UNIVERSAL>{(T)a.wmin, one_minus_eps2<T>(), (const T*)a.c_dev});
+    case GM_GRASSMANN:
+      if (a.p == 2 && (a.flags & GM_FAST_SVD)) return launch_grassmann<T, 2, true>(a, grid, block);
+      switch (a.p) {
+        case 1: return launch_grassmann<T, 1, false>(a, grid, block);
+        case 2: return launch_grassmann<T, 2, false>(a, grid, block);
+        case 3: return launch_grassmann<T, 3, false>(a, grid, block);
+        case 4: return launch_grassmann<T, 4, false>(a, grid, block);
+        case 5: return launch_grassmann<T, 5, false>(a, grid, block);
+        default: return GM_EUNSUPPORTED;
+      }
+    default: return GM_EINVAL;
   }
-  note_launch();
-  return check_launch();
 }
 
 int vec_launch(const PairArgs& a) {
