@@ -94,6 +94,9 @@ class PairSet:
             raise ValueError('sampled pairs: int32 CUDA sources and a uint8 (S, N) level matrix')
         if slots is not None and (slots.dtype != torch.int32 or slots.numel() != sources.numel()):
             raise ValueError('sampled pairs: slots must be int32, one per source')
+        if slots is None and sources.numel() > levels.shape[0]:
+            raise ValueError('sampled pairs: without slots, source g reads row g of the level matrix: more sources '
+                             'than rows')
         n = levels.shape[1]
         if n >= (1 << 24):
             raise ValueError('sampled pairs need fewer than 2^24 nodes')

@@ -11,8 +11,6 @@ ranks, ONE fused optimizer kernel.  The semantics of a step are exactly those of
 
 with the reference's manifold / objective / optimizer definitions.
 """
-import os
-
 import torch
 from torch.nn.functional import softplus
 
@@ -90,6 +88,95 @@ def pack_hops2(offsets, idx_j, hops):
     return words.contiguous(), bases.contiguous(), order
 
 
+def _named(**tensors):
+    return {name: t for name, t in tensors.items() if t is not None}
+
+
+def _grouped_upload(sources, offsets, idx_j, hops=None, bases=None):
+    """The host tensors of a source-grouped batch that go to the device (the bases only with 2-byte words)."""
+    two_byte = hops is None and idx_j.dtype == torch.int16
+    if two_byte and bases is None:
+        raise ValueError('2-byte pair words need the bases vector of pack_hops2')
+    return _named(sources=sources, offsets=offsets, j=idx_j, hops=hops, bases=bases if two_byte else None)
+
+
+class _UploadRing:
+    """Device copies of the pinned host tensors of a training step, with the next step's copy overlapped on a second
+    stream.  Two slots of grow-only byte buffers, one per tensor name, viewed as each batch's dtypes: while a step reads
+    one slot, the next batch is copied into the other.  Each slot keeps the event of its last copy-stream upload, and
+    the compute stream waits on it before the slot is rewritten or its buffers are replaced, so a prefetched batch that
+    the next step does not take, or a batch larger than any before, never races the copy stream.  All buffers are
+    allocated on the compute stream."""
+
+    def __init__(self, device):
+        self.device = device
+        self.stream = torch.cuda.Stream(device=device)
+        self.slots = [{}, {}]
+        self.events = [None, None]
+        self.current = 0  # slot the current step reads
+        self.pending = None  # (batch, slot) of the prefetch the next take() may claim
+        self.outputs = {}  # outputs of the expansion kernels: written and read on the compute stream only
+
+    def _buffer(self, bufs, name, numel, dtype):
+        n = numel * dtype.itemsize
+        if name not in bufs or bufs[name].numel() < n:
+            bufs[name] = torch.empty(max(n, 1), dtype=torch.uint8, device=self.device)
+        return bufs[name][:n].view(dtype)
+
+    def _claim(self, slot):
+        """Views of the slot's buffers may be rewritten or replaced on the compute stream after this."""
+        if self.events[slot] is not None:
+            torch.cuda.current_stream(self.device).wait_event(self.events[slot])
+            self.events[slot] = None
+
+    def _views(self, slot, batch):
+        return {name: self._buffer(self.slots[slot], name, t.numel(), t.dtype) for name, t in batch.items()}
+
+    def take(self, batch):
+        """Device views of `batch` (name -> pinned host tensor) for a step on the current stream: the prefetched
+        slot if prefetch() was given these very tensors, else a copy on the current stream."""
+        pending, self.pending = self.pending, None
+        if (pending is not None and pending[0].keys() == batch.keys()
+                and all(pending[0][name] is t for name, t in batch.items())):
+            self.current = pending[1]
+            self._claim(self.current)
+            return self._views(self.current, batch)
+        self.current = 0
+        self._claim(0)
+        views = self._views(0, batch)
+        for name, t in batch.items():
+            views[name].copy_(t, non_blocking=True)
+        return views
+
+    def prefetch(self, batch):
+        """Copy the next step's `batch` on the copy stream into the slot the current step does not read."""
+        slot = 1 - self.current
+        self._claim(slot)
+        views = self._views(slot, batch)
+        self.stream.wait_stream(torch.cuda.current_stream(self.device))  # earlier steps are done with the slot
+        with torch.cuda.stream(self.stream):
+            for name, t in batch.items():
+                views[name].copy_(t, non_blocking=True)
+        self.events[slot] = self.stream.record_event()
+        self.pending = (batch, slot)
+
+    def output(self, name, numel):
+        """int32 (numel,) device buffer for the output of an expansion kernel."""
+        return self._buffer(self.outputs, name, numel, torch.int32)
+
+
+def _replace_param(optimizer, old, new):
+    """Let the optimizer drive `new` wherever it holds the embedding parameter `old`."""
+    replaced = False
+    for g in optimizer.param_groups:
+        for k, prm in enumerate(g['params']):
+            if prm is old:
+                g['params'][k] = new
+                replaced = True
+    if not replaced:
+        raise ValueError('optimizer does not hold the embedding parameter')
+
+
 class PairTrainer:
     """Drives (I, J, hops) pair batches through a single-manifold embedding.
 
@@ -121,12 +208,9 @@ class PairTrainer:
         self.grad = torch.zeros_like(self.x, memory_format=torch.contiguous_format)
         self.x.grad = self.grad
         self.acc = torch.zeros(2, dtype=torch.float64, device=self.x.device)
-        self._staging = None
-        self._copy_stream = None
+        self._ring = _UploadRing(self.x.device)
         self.shards = None
         self.peer = None
-        self._grad_is_clean = False
-        self._fold_zero_grad = False
         if process_group is not None and torch.distributed.get_world_size(process_group) > 1:
             even = self.x.shape[0] % torch.distributed.get_world_size(process_group) == 0
             if owner_update is None:
@@ -150,21 +234,7 @@ class PairTrainer:
                 else:
                     own.grad = torch.zeros_like(own.data)
                 self._own = own
-                replaced = False
-                for g in optimizer.param_groups:
-                    for k, prm in enumerate(g['params']):
-                        if prm is self.x:
-                            g['params'][k] = own
-                            replaced = True
-                if not replaced:
-                    raise ValueError('optimizer does not hold the embedding parameter')
-        if self.shards is None and os.environ.get('GM_FOLD_ZERO_GRAD', '0') == '1':
-            # the trainer owns the gradient buffer, so the optimizer kernel can hand every row back zeroed
-            # (gm_optim_t.zero_grad) instead of a full-table memset at the top of the next step.  OFF by default:
-            # measured on B200 (2 M SPD4 points) the step is 1.28 ms with it and 1.19 ms with the memset -- the
-            # memset leaves the 128 MB table L2-resident for the pair kernel's reductions, the fused zeroing does not
-            self.x._gm_zero_grad_after_step = True
-            self._fold_zero_grad = True
+                _replace_param(optimizer, self.x, own)
 
     # ---- device-resident inputs ---------------------------------------------------------------------------------
     def step(self, idx_i, idx_j, hops, epoch=1, segments=0):
@@ -194,18 +264,8 @@ class PairTrainer:
         """step_sampled from PINNED host tensors: `sources` (and `slots`) int32 (G,) are the step's whole upload --
         8 bytes per source instead of 4-9 bytes per pair.  Returns the loss as a Python float (a device->host read), or
         with defer_loss=True the loss of the previous deferred step (see step_host_grouped)."""
-        G = sources.numel()
-        dev = self.x.device
-        if getattr(self, '_src_staging', None) is None or self._src_staging[0][0].numel() < G:
-            self._src_staging = [(torch.empty(G, dtype=torch.int32, device=dev),
-                                  torch.empty(G, dtype=torch.int32, device=dev)) for _ in range(2)]
-            self._src_slot = 0
-        ds, dl = self._src_staging[self._src_slot]
-        self._src_slot ^= 1  # the other buffer may still be read by the previous step's kernel
-        ds[:G].copy_(sources, non_blocking=True)
-        if slots is not None:
-            dl[:G].copy_(slots, non_blocking=True)
-        loss = self.step_sampled(ds[:G], levels, per_src, seed, slots=None if slots is None else dl[:G], epoch=epoch)
+        d = self._ring.take(_named(sources=sources, slots=slots))
+        loss = self.step_sampled(d['sources'], levels, per_src, seed, slots=d.get('slots'), epoch=epoch)
         if defer_loss:
             return self._queue_loss_read()
         return loss.item()
@@ -232,8 +292,9 @@ class PairTrainer:
 
     def _step_pairs(self, pairs, targets, epoch):
         loss_spec = self.obj.loss_spec(epoch=epoch, alpha=self.alpha)
-        if not self._grad_is_clean:
-            self.grad.zero_()
+        # a memset rather than rows handed back zeroed by the optimizer kernel (gm_optim_t.zero_grad): measured on B200
+        # (2 M SPD4 points) 1.19 vs 1.28 ms per step, the memset leaves the table L2-resident for the pair kernel
+        self.grad.zero_()
         self.acc.zero_()
         if self.deterministic:
             self._pairs_deterministic(pairs, targets, loss_spec, _softplus_value(self.emb.scales[0]))
@@ -244,7 +305,6 @@ class PairTrainer:
                 raise RuntimeError('deterministic accumulation: single GPU, or the peer-memory owner update (which '
                                    'sums the ranks in rank order)')
             self.opt.step()
-            self._grad_is_clean = self._fold_zero_grad
             return self.acc[0]
         # softplus(scale) is re-read every step (cached on the parameter until somebody steps it or loads a snapshot);
         # the trainer itself does not train the scale: acc[1] (sum l' d2) is there for a caller who does
@@ -264,8 +324,6 @@ class PairTrainer:
         if self.shards is None:
             allreduce_step_buffers(self.grad, self.acc, self.pg)
             self.opt.step()
-            # single GPU / replicated update: the optimizer kernel zeroed every gradient row after reading it
-            self._grad_is_clean = self._fold_zero_grad
         else:
             self.shards.reduce_scatter(self.grad, out=self._own.grad)
             torch.distributed.all_reduce(self.acc, group=self.pg)
@@ -274,52 +332,14 @@ class PairTrainer:
         return self.acc[0]
 
     # ---- host-resident inputs (what a data loader hands over) ----------------------------------------------------------
-    def _ensure_staging(self, P, hop_dtype, G=0):
-        if (self._staging is None or self._staging[0][0].numel() < P or self._staging[0][3].numel() < G
-                or self._staging[0][2].dtype != hop_dtype):
-            dev = self.x.device
-            self._staging = [(torch.empty(P, dtype=torch.int32, device=dev), torch.empty(P, dtype=torch.int32, device=dev),
-                              torch.empty(P, dtype=hop_dtype, device=dev), torch.empty(max(G, 1), dtype=torch.int32, device=dev),
-                              torch.empty(max(G, 1) + 1, dtype=torch.int64, device=dev)) for _ in range(2)]
-            self._copy_stream = torch.cuda.Stream(device=dev)
-            self._slot = 0
-            self._pending = None
-
     def step_host(self, idx_i, idx_j, hops, epoch=1, next_batch=None):
         """One step from PINNED host tensors (int32 indices, uint8/int16 hop counts).  Copies the batch to the device,
         runs the step and returns the loss as a Python float (a device->host read).  If `next_batch` (a tuple of
         pinned host tensors) is given its upload is overlapped with this step's kernels on a second stream."""
-        P = idx_i.numel()
-        self._ensure_staging(P, hops.dtype)
-        cur = torch.cuda.current_stream(self.x.device)
-        if self._pending is not None and self._pending[0] is idx_i:
-            slot, ev = self._pending[1], self._pending[2]
-            cur.wait_event(ev)
-        else:
-            slot = self._slot
-            di, dj, dh = self._staging[slot][:3]
-            di[:P].copy_(idx_i, non_blocking=True)
-            dj[:P].copy_(idx_j, non_blocking=True)
-            dh[:P].copy_(hops, non_blocking=True)
-        di, dj, dh = self._staging[slot][:3]
-        self._pending = None
+        d = self._ring.take(_named(i=idx_i, j=idx_j, hops=hops))
         if next_batch is not None:
-            nslot = 1 - slot
-            ni, nj, nh = self._staging[nslot][:3]
-            n = next_batch[0].numel()
-            if n > ni.numel() or next_batch[2].dtype != nh.dtype:
-                raise ValueError('next_batch does not fit the staging buffers (more pairs, or another hop dtype, than '
-                                 'the batch of this step)')
-            self._copy_stream.wait_stream(cur)  # the other slot was consumed by the previous step
-            with torch.cuda.stream(self._copy_stream):
-                ni[:n].copy_(next_batch[0], non_blocking=True)
-                nj[:n].copy_(next_batch[1], non_blocking=True)
-                nh[:n].copy_(next_batch[2], non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(self._copy_stream)
-            self._pending = (next_batch[0], nslot, ev)
-        self._slot = 1 - slot
-        loss = self.step(di[:P], dj[:P], dh[:P], epoch=epoch)
+            self._ring.prefetch(_named(i=next_batch[0], j=next_batch[1], hops=next_batch[2]))
+        loss = self.step(d['i'], d['j'], d['hops'], epoch=epoch)
         return loss.item()
 
     # ---- pipelined loss read-back --------------------------------------------------------------------------------
@@ -360,71 +380,24 @@ class PairTrainer:
         enqueue step k+1 while the GPU runs step k.
         Two bytes per pair: idx_j = the int16 words of pack_hops2 (every group's targets sorted by row, stored as
         gaps), hops=None, bases = its int32 (G,) vector; `next_batch` then carries the bases as a fifth entry."""
+        batch = _grouped_upload(sources, offsets, idx_j, hops, bases)
+        nxt = None if next_batch is None else _grouped_upload(*next_batch)
         packed3 = hops is None and idx_j.dtype == torch.uint8  # pack_hops3: 3 bytes per pair over PCIe
         packed2 = hops is None and idx_j.dtype == torch.int16  # pack_hops2: 2 bytes per pair
-        if packed2 and bases is None:
-            raise ValueError('2-byte pair words need the bases vector of pack_hops2')
-        P, G = (int(offsets[-1]) if packed3 else idx_j.numel()), sources.numel()
-        packed = hops is None  # idx_j carries the hop counts (pack_hops / pack_hops3)
-        self._ensure_staging(P, torch.uint8 if packed else hops.dtype, G)
-        if packed3 and (getattr(self, '_staging3', None) is None or self._staging3[0].numel() < idx_j.numel()):
-            self._staging3 = [torch.empty(idx_j.numel(), dtype=torch.uint8, device=self.x.device) for _ in range(2)]
-        if packed2 and (getattr(self, '_staging2', None) is None or self._staging2[0][0].numel() < P
-                        or self._staging2[0][1].numel() < G):
-            self._staging2 = [(torch.empty(P, dtype=torch.int16, device=self.x.device),
-                               torch.empty(max(G, 1), dtype=torch.int32, device=self.x.device)) for _ in range(2)]
-        cur = torch.cuda.current_stream(self.x.device)
-
-        def upload(slot, batch):
-            di, dj, dh, ds, do = self._staging[slot]
-            s_, o_, j_, h_ = batch[:4]
-            if j_.dtype == torch.int16:  # 2-byte words + bases: staged raw, expanded on the device before the step
-                w2, b2 = self._staging2[slot]
-                if s_.numel() > ds.numel() or j_.numel() > w2.numel() or len(batch) < 5 or batch[4].numel() > b2.numel():
-                    raise ValueError('batch does not fit the staging buffers of the first batch of this call')
-                ds[:s_.numel()].copy_(s_, non_blocking=True)
-                do[:o_.numel()].copy_(o_, non_blocking=True)
-                w2[:j_.numel()].copy_(j_, non_blocking=True)
-                b2[:batch[4].numel()].copy_(batch[4], non_blocking=True)
-                return
-            jcap = self._staging3[slot].numel() if j_.dtype == torch.uint8 else dj.numel()
-            if s_.numel() > ds.numel() or j_.numel() > jcap or (h_ is not None and h_.dtype != dh.dtype):
-                raise ValueError('batch does not fit the staging buffers (more sources / pairs, or another hop dtype, '
-                                 'than the first batch of this call)')
-            ds[:s_.numel()].copy_(s_, non_blocking=True)
-            do[:o_.numel()].copy_(o_, non_blocking=True)
-            if j_.dtype == torch.uint8:  # 3-byte words: staged raw, expanded on the device just before the step
-                self._staging3[slot][:j_.numel()].copy_(j_, non_blocking=True)
-            else:
-                dj[:j_.numel()].copy_(j_, non_blocking=True)
-            if h_ is not None:
-                dh[:h_.numel()].copy_(h_, non_blocking=True)
-
-        if self._pending is not None and self._pending[0] is idx_j:
-            slot, ev = self._pending[1], self._pending[2]
-            cur.wait_event(ev)
-        else:
-            slot = self._slot
-            upload(slot, (sources, offsets, idx_j, hops, bases))
-        di, dj, dh, ds, do = self._staging[slot]
-        self._pending = None
-        if next_batch is not None:
-            nslot = 1 - slot
-            self._copy_stream.wait_stream(cur)  # the other slot was consumed by the previous step
-            with torch.cuda.stream(self._copy_stream):
-                upload(nslot, next_batch)
-                ev = torch.cuda.Event()
-                ev.record(self._copy_stream)
-            self._pending = (next_batch[2], nslot, ev)
-        self._slot = 1 - slot
+        P = int(offsets[-1]) if packed3 else idx_j.numel()
+        d = self._ring.take(batch)
+        if nxt is not None:
+            self._ring.prefetch(nxt)
+        di = self._ring.output('i', P)
         if packed2:  # one kernel: gaps -> rows (segmented scan per group) and the group's first endpoint per pair
-            w2, b2 = self._staging2[slot]
-            _ops.unpack_pairs2(w2[:P], b2[:G], do[:G + 1], dj, group_rows=ds[:G], out_i=di)
+            dj = self._ring.output('j', P)
+            _ops.unpack_pairs2(d['j'], d['bases'], d['offsets'], dj, group_rows=d['sources'], out_i=di)
         else:
-            _ops.expand_groups(ds[:G], do[:G + 1], di[:P])
-        if packed3:
-            _ops.unpack_pairs3(self._staging3[slot], P, dj)
-        loss = self.step(di[:P], dj[:P], None if packed else dh[:P], epoch=epoch, segments=segments)
+            _ops.expand_groups(d['sources'], d['offsets'], di)
+            dj = d['j']
+        if packed3:  # 3-byte words: staged raw, expanded on the device just before the step
+            dj = _ops.unpack_pairs3(d['j'], P, self._ring.output('j', P))
+        loss = self.step(di, dj, d.get('hops'), epoch=epoch, segments=segments)
         if defer_loss:  # read this step's loss back asynchronously, hand out the previous step's
             return self._queue_loss_read()
         return loss.item()
@@ -476,22 +449,12 @@ class ShardedPairTrainer(PairTrainer):
         own.grad = arena.grad
         own._gm_zero_grad_after_step = True  # the local optimizer kernel hands every gradient row back zeroed
         self._own = own
-        replaced = False
-        for g in optimizer.param_groups:
-            for k, prm in enumerate(g['params']):
-                if prm is full:
-                    g['params'][k] = own
-                    replaced = True
-        if not replaced:
-            raise ValueError('optimizer does not hold the embedding parameter')
+        _replace_param(optimizer, full, own)
         self._full = full
         if not keep_full:
             full.data = full.data.new_empty((0,) + tuple(full.shape[1:]))
-        self._staging = None
-        self._copy_stream = None
+        self._ring = _UploadRing(self.x.device)
         self.shards = None
-        self._grad_is_clean = True
-        self._fold_zero_grad = True
 
     def _step_pairs(self, pairs, targets, epoch):
         loss_spec = self.obj.loss_spec(epoch=epoch, alpha=self.alpha)

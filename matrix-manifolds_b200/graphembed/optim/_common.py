@@ -21,7 +21,7 @@ def spec_of(param):
 def fused_step(param, grad, cfg, buf1=None, buf2=None):
     spec, manifold = spec_of(param)
     cfg.grassmann_retr_qr = int(getattr(manifold, 'retr_kind', 'svd') == 'qr')
-    # a training loop that owns the gradient buffer (engine.PairTrainer) lets the update kernel hand it back zeroed
+    # a training loop that owns the gradient buffer (engine.ShardedPairTrainer) lets the update kernel hand it back zeroed
     cfg.zero_grad = int(getattr(param, '_gm_zero_grad_after_step', False) and grad.is_contiguous()
                         and grad.dtype == param.dtype)
     with torch.no_grad():

@@ -398,17 +398,16 @@ def test_lean_step_equals_autograd_step_for_products(kind, tmp_path):
     assert abs(outs[0][2][0].item() - start) > 1e-7  # scale / curvature parameters really were trained
 
 
-def test_pair_trainer_folded_zero_grad_matches_explicit_memset(monkeypatch):
-    """PairTrainer lets the optimizer kernel clear every gradient row it has read (gm_optim_t.zero_grad) instead of
-    zeroing the table at the top of the next step: 4 steps against the explicit zero -> pairs -> update sequence."""
+def test_optimizer_zero_grad_after_step_matches_explicit_memset():
+    """RiemannianAdam on a parameter marked _gm_zero_grad_after_step (what ShardedPairTrainer sets) lets the optimizer
+    kernel clear every gradient row it has read (gm_optim_t.zero_grad), so the gradient buffer is zeroed once before
+    the first step only: 4 pair-kernel + optimizer steps against the explicit zero -> pairs -> update sequence."""
     from graphembed import _ops, _lib as L
-    from graphembed.engine import PairTrainer
     from graphembed.manifolds import SymmetricPositiveDefinite
     from graphembed.modules import ManifoldEmbedding
     from graphembed.objectives import QuotientLoss
     from graphembed.optim import RiemannianAdam
     n, P = 3000, 50000
-    monkeypatch.setenv('GM_FOLD_ZERO_GRAD', '1')
     g = torch.Generator().manual_seed(9)
     batches = []
     for _ in range(4):
@@ -417,15 +416,23 @@ def test_pair_trainer_folded_zero_grad_matches_explicit_memset(monkeypatch):
         batches.append((I.to(DEV), J.to(DEV), torch.randint(1, 9, (P,), generator=g, dtype=torch.uint8).to(DEV)))
     torch.manual_seed(5)
     emb = ManifoldEmbedding(n, [SymmetricPositiveDefinite(4)], device=DEV, dtype=torch.float64)
-    x_ref = emb.xs[0].detach().clone()
-    tr = PairTrainer(emb, RiemannianAdam(emb.xs, lr=0.01, max_grad_norm=100, exact=True), QuotientLoss(), max_hops_sq=64.0)
-    assert tr._fold_zero_grad
-    losses = [tr.step(*b, epoch=k + 1).item() for k, b in enumerate(batches)]
-    assert float(tr.grad.abs().max().item()) == 0.0  # handed back cleared
-    # explicit sequence on a copy
     man = emb.manifolds[0]
-    m, v = torch.zeros_like(x_ref), torch.zeros_like(x_ref)
+    x = emb.xs[0]
+    x_ref = x.detach().clone()
     sp = float(torch.nn.functional.softplus(torch.tensor(0.5)))
+    x.grad = torch.zeros_like(x)
+    x._gm_zero_grad_after_step = True
+    opt = RiemannianAdam(emb.xs, lr=0.01, max_grad_norm=100, exact=True)
+    losses = []
+    for k, (I, J, H) in enumerate(batches):
+        acc, _ = _ops.pairs_loss_fused(man.spec, x.detach(), _ops.PairSet.from_lists(I, J, DEV),
+                                       _ops.TargetSpec.hops(H, 64.0), QuotientLoss().loss_spec(epoch=k + 1, alpha=1.0),
+                                       sp, x.grad)
+        losses.append(acc[0].item())
+        opt.step()
+        assert float(x.grad.abs().max().item()) == 0.0  # handed back cleared
+    # explicit sequence on a copy
+    m, v = torch.zeros_like(x_ref), torch.zeros_like(x_ref)
     ref_losses = []
     for k, (I, J, H) in enumerate(batches):
         grad = torch.zeros_like(x_ref)

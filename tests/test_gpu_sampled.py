@@ -75,6 +75,10 @@ def test_validation_of_sampled_pairs():
                               torch.zeros_like(x))
     with pytest.raises(ValueError):
         _ops.PairSet.sampled(src.long(), lv, 8, 1)
+    with pytest.raises(ValueError):  # source 4 would read row 4 of a 4-row level matrix
+        _ops.PairSet.sampled(torch.arange(5, dtype=torch.int32, device=DEV), lv, 8, 1)
+    _ops.PairSet.sampled(torch.arange(5, dtype=torch.int32, device=DEV), lv, 8, 1,
+                         slots=torch.zeros(5, dtype=torch.int32, device=DEV))
 
 
 def test_step_sampled_is_the_step_on_the_host_drawn_lists():
