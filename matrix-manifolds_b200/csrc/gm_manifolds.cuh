@@ -224,14 +224,15 @@ struct SpdAI {
     GM_UNROLL for (int i = 0; i < N; ++i)
       GM_UNROLL for (int j = 0; j <= i; ++j) ap[i * (i + 1) / 2 + j] = ic.a[i * N + j];
   }
-  // max_sweeps / converged: see jacobi_eigh.  With the default cap `converged` is of no interest.
+  // max_sweeps / converged / PACK: see jacobi_eigh.  With the default cap `converged` is of no interest.
+  template <bool PACK = false>
   GM_HD T eig_forward(const T (&a)[E], const T (&y)[E], EigState& st, int max_sweeps = JacobiCfg<T>::max_sweeps,
                       bool* converged = nullptr) const {
     T m[E], w[N];
     congr_lower<T, N>(a, y, m);
     GM_UNROLL for (int i = 0; i < N; ++i)
       GM_UNROLL for (int j = 0; j < N; ++j) st.wm[i * N + j] = (j >= i) ? a[j * N + i] : (T)0;
-    const bool conv = jacobi_eigh<T, N, true, false>(m, st.wm, w, max_sweeps);
+    const bool conv = jacobi_eigh<T, N, true, false, PACK>(m, st.wm, w, max_sweeps);
     if (converged) *converged = conv;
     T phi = (T)0;
     // log_pos needs a positive normal finite argument: guaranteed by the clamp for every sane [wmin, wmax]
@@ -247,12 +248,13 @@ struct SpdAI {
     }
     return clamp_min(phi, wmin);
   }
+  template <bool PACK = false>
   GM_HD T eig_forward_prepped(const T (&ap)[kPrepSize], const T (&y)[E], EigState& st,
                               int max_sweeps = JacobiCfg<T>::max_sweeps, bool* converged = nullptr) const {
     T a[E];
     GM_UNROLL for (int i = 0; i < N; ++i)
       GM_UNROLL for (int j = 0; j < N; ++j) a[i * N + j] = (j <= i) ? ap[i * (i + 1) / 2 + j] : (T)0;
-    return eig_forward(a, y, st, max_sweeps, converged);
+    return eig_forward<PACK>(a, y, st, max_sweeps, converged);
   }
   GM_HD void eig_backward(const EigState& st, T wgt, T (&gx)[E], T (&gy)[E]) const {
     T cx[N], cy[N];
@@ -331,6 +333,7 @@ struct SpdStein {
   T wmin, wmax;
   struct EigState {};
   GM_HD void prep(const T (&)[E], T (&)[1]) const {}
+  template <bool PACK = false>
   GM_HD T eig_forward_prepped(const T (&)[1], const T (&)[E], EigState&, int = 0, bool* = nullptr) const { return (T)0; }
   GM_HD void eig_backward(const EigState&, T, T (&)[E], T (&)[E]) const {}
 

@@ -174,6 +174,54 @@ template <> struct Num<double> {
   GM_HD static double copysign(double a, double b) { return ::copysign(a, b); }
 };
 
+// ---------------------------------------------------------------------------
+// Two independent scalar operations as one packed FP32x2 instruction (FFMA2 / FMUL2 on sm_100a; ptxas does not pair
+// scalar ones by itself).  Each lane rounds exactly as the scalar instruction does, so every helper returns the bits
+// of the scalar form named next to it -- the form the compiler already contracts the plain expression to
+// (a * b - c * d is fma(a, b, -(c * d))).  double and the host build (tests/hostcheck) evaluate the plain expression.
+// ---------------------------------------------------------------------------
+template <typename T> struct Two { T x, y; };
+
+// (a.x b.x + c.x, a.y b.y + c.y), one rounding per lane (s += a * b after the compiler's contraction)
+template <typename T>
+GM_HD Two<T> fma2(Two<T> a, Two<T> b, Two<T> c) {
+#ifdef __CUDA_ARCH__
+  if constexpr (sizeof(T) == 4) {
+    const float2 r = __ffma2_rn(make_float2(a.x, a.y), make_float2(b.x, b.y), make_float2(c.x, c.y));
+    return {r.x, r.y};
+  }
+#endif
+  return {a.x * b.x + c.x, a.y * b.y + c.y};
+}
+// (a.x b.x, a.y b.y)
+template <typename T>
+GM_HD Two<T> mul2(Two<T> a, Two<T> b) {
+#ifdef __CUDA_ARCH__
+  if constexpr (sizeof(T) == 4) {
+    const float2 r = __fmul2_rn(make_float2(a.x, a.y), make_float2(b.x, b.y));
+    return {r.x, r.y};
+  }
+#endif
+  return {a.x * b.x, a.y * b.y};
+}
+// Plane rotation of the coordinate pairs (p0, q0) and (p1, q1):  p <- c p - s q = fma(c, p, -(s q)),
+// q <- s p + c q = fma(s, p, c q).
+template <typename T>
+GM_HD void rot2(T c, T s, T& p0, T& q0, T& p1, T& q1) {
+#ifdef __CUDA_ARCH__
+  if constexpr (sizeof(T) == 4) {
+    const Two<T> cc{c, c}, p{p0, p1}, q{q0, q1};
+    const Two<T> sq = mul2(Two<T>{s, s}, q);
+    const Two<T> np = fma2(cc, p, Two<T>{-sq.x, -sq.y});
+    const Two<T> nq = fma2(Two<T>{s, s}, p, mul2(cc, q));
+    p0 = np.x; p1 = np.y; q0 = nq.x; q1 = nq.y;
+    return;
+  }
+#endif
+  const T np0 = c * p0 - s * q0, nq0 = s * p0 + c * q0;
+  const T np1 = c * p1 - s * q1, nq1 = s * p1 + c * q1;
+  p0 = np0; q0 = nq0; p1 = np1; q1 = nq1;
+}
 // torch.clamp semantics on a *value* (NaN propagates like torch: clamp(NaN)=NaN)
 template <typename T>
 GM_HD T clampv(T x, T lo, T hi) {
@@ -360,7 +408,12 @@ struct JacobiFirstCheck { static constexpr int value = N >= 4 ? 3 : (N == 3 ? 2 
 // max_sweeps (<= JacobiCfg<T>::max_sweeps) caps the number of sweeps; the return value says whether the convergence
 // test passed (always evaluated once the cap is reached, so a caller can run a fixed number of sweeps and hand the
 // few matrices that need more to a second pass -- the streaming pair kernel does, see gm_pairs_spd.cu).
-template <typename T, int N, bool WANT_V = true, bool INIT_V = true>
+// PACK: rotate the eigenvector row pairs (0, 1), (2, 3), ... together (rot2: FMUL2 + FFMA2 in fp32, the same bits
+// as the scalar form).  Only the window-ordered SPEC pair kernel sets it, where it measured 0.901 -> 0.854 ms
+// (profiles/r03_packed_rotations_ab.txt).  The general 4x4 stream instantiation measured 2.7 % SLOWER with it
+// (1.019 -> 1.047 ms, --windows 0) although it issued fewer instructions and used one register fewer, so every other
+// caller keeps the scalar rotation.
+template <typename T, int N, bool WANT_V = true, bool INIT_V = true, bool PACK = false>
 GM_HD bool jacobi_eigh(T (&a)[N * N], T (&v)[N * N], T (&w)[N], int max_sweeps = JacobiCfg<T>::max_sweeps) {
   if (WANT_V && INIT_V) {
     GM_UNROLL for (int i = 0; i < N; ++i)
@@ -386,6 +439,8 @@ GM_HD bool jacobi_eigh(T (&a)[N * N], T (&v)[N * N], T (&w)[N], int max_sweeps =
     }
     a[p * N + q] = (T)0;
     a[q * N + p] = (T)0;
+    // Rows of `a` stay scalar even with PACK: their row pairs change from rotation to rotation, and packing them cost
+    // as many register moves as it saved FMAs (N = 4 SPEC kernel: +24 MOV for -24 FFMA/FMUL).
     GM_UNROLL for (int r = 0; r < N; ++r) {
       if (r != p && r != q) {
         T arp = a[r * N + p], arq = a[r * N + q];
@@ -395,7 +450,11 @@ GM_HD bool jacobi_eigh(T (&a)[N * N], T (&v)[N * N], T (&w)[N], int max_sweeps =
         a[r * N + q] = nrq; a[q * N + r] = nrq;
       }
     }
-    if (WANT_V) {
+    if constexpr (WANT_V && PACK) {
+      static_assert(N % 2 == 0, "PACK rotates whole row pairs");
+      GM_UNROLL for (int r = 0; r < N; r += 2)
+        rot2(c, s, v[r * N + p], v[r * N + q], v[(r + 1) * N + p], v[(r + 1) * N + q]);
+    } else if (WANT_V) {
       GM_UNROLL for (int r = 0; r < N; ++r) {
         T vrp = v[r * N + p], vrq = v[r * N + q];
         v[r * N + p] = c * vrp - s * vrq;

@@ -419,7 +419,7 @@ spd_pair_stream_kernel(Op op, PairSpec ps, const T* __restrict__ xa, const T* __
       [[maybe_unused]] typename Op::EigState st;
       if constexpr (Op::kCanPrep) {
         if (ra0 != prep_row) { op.prep(x, ap); prep_row = ra0; }
-        d2 = op.eig_forward_prepped(ap, y, st);
+        d2 = op.template eig_forward_prepped<SPEC != 0>(ap, y, st);  // SPEC: packed eigenvector rotations
       } else {
         d2 = op.dist2_grad(x, y, gx, gy);
       }
